@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- Hap frame encode/decode throughput of libhap_b200.so (contract: see the task brief).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload 4k_hapq|16k_stream]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload 4k_hapq|16k_stream] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json `metric` "4K Hap-Q encode/decode GB/s per GPU", configs[2]): 3840x2160 RGBA8
 synthetic video frames -> Hap Q (scaled-YCoCg-DXT5, Snappy, 8 chunks) -> decoded back to the DXT texture bytes
@@ -331,6 +331,31 @@ def extra_config_lines(lib, torch, dev, peak):
     return out
 
 
+DUMP_SAMPLE = 1 << 22     # bytes sampled from the encoded frames and from the decoded textures: 16 MB of float32 each
+
+
+def dump_outputs(out_dir, frames, used, cap, tex, tex_bytes):
+    """--dump-outputs: what the last timed step handed back -- every frame's encoded length (frame_lengths.npy, float64), and
+    a fixed, seeded sample of the encoded frame bytes (frame_bytes_sample.npy; -1 where a sampled position lies past its
+    frame's end) and of the decoded texture bytes (texture_bytes_sample.npy), float32.  The inputs are seeded too, so two
+    builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = used.numel()
+    rng = np.random.default_rng(0)
+    dev = frames.device
+    pos = torch.from_numpy(np.sort(rng.integers(0, n * cap, DUMP_SAMPLE))).to(dev)
+    fb = frames.view(-1)[pos].float()
+    fb[(pos % cap) >= used[pos // cap]] = -1.0
+    pos = torch.from_numpy(np.sort(rng.integers(0, n * tex_bytes, DUMP_SAMPLE))).to(dev)
+    stride = (tex_bytes + 15) // 16 * 16
+    tb = tex.view(-1)[(pos // tex_bytes) * stride + pos % tex_bytes].float()
+    np.save(os.path.join(out_dir, "frame_lengths.npy"), used.double().cpu().numpy())
+    np.save(os.path.join(out_dir, "frame_bytes_sample.npy"), fb.cpu().numpy())
+    np.save(os.path.join(out_dir, "texture_bytes_sample.npy"), tb.cpu().numpy())
+
+
 def run_gpu_arm(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -430,6 +455,9 @@ def run_gpu_arm(args, rank, local_rank, world):
         launches = lib.launches() - launches0
         clocks = sampler.stop(wall0, wall1) if rank == 0 else None
         A.check()
+        if args.dump_outputs and rank == 0:
+            last = (state["n"] - 1) & 1
+            dump_outputs(args.dump_outputs, frames_buf[last], used[last], A.cap, A.tex[0], A.tex_bytes[0])
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -814,7 +842,13 @@ def main():
     ap.add_argument("--profile", action="store_true", help="short run for ncu: skip the e2e, extra and CPU legs")
     ap.add_argument("--no-overlap", action="store_true", help="encode and decode of a batch back to back on one stream")
     ap.add_argument("--no-index", action="store_true", help="frames without the trailing fragment index section (decoder indexes on the fly)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed (encoded frame "
+                                                          "lengths, sampled frame and texture bytes) as .npy files into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "4k_hapq"):
+        ap.error("--dump-outputs applies to the 4k_hapq workload of the b200 implementation")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

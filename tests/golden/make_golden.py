@@ -22,6 +22,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import oracles  # noqa: E402
+from golden_util import cpu_differential_case, gpu_differential_case, pack_frame  # noqa: E402
 from hap_b200 import synth  # noqa: E402
 from hap_b200.abi import (HapCompressorNone, HapCompressorSnappy, HapTextureFormat_A_RGTC1,  # noqa: E402
                           HapTextureFormat_RGB_DXT1, HapTextureFormat_RGBA_DXT5, HapTextureFormat_YCoCg_DXT5)
@@ -218,6 +219,41 @@ def main():
     enc["two_dxt1"] = ref.encode([p16, p16], [DXT1, DXT1], [1, 1], [1, 1])[0]
     enc["ycocg_plus_dxt1"] = ref.encode([p16, p16], [YCOCG, DXT1], [1, 1], [1, 1])[0]
     G["encode_results"] = enc
+
+    # ---- seeded differential cases: the reference's frames of each payload (None and Snappy), and its decode of the
+    #      oracle's Snappy frame of the same payload
+    orc = oracles.oracle_abi()
+    diff = {}
+    for seed in range(6):
+        payload, fmt, k = cpu_differential_case(seed)
+        rn, fn = ref.encode([payload], [fmt], [HapCompressorNone], [k])
+        rs, fs = ref.encode([payload], [fmt], [HapCompressorSnappy], [k])
+        ro, fo = orc.encode([payload], [fmt], [HapCompressorSnappy], [k])
+        rd, data, dfmt, _ = ref.decode(fo, 0, len(payload))
+        diff[str(seed)] = {"max_len": ref.max_encoded_length([len(payload)], [fmt], [k]),
+                           "none": {"result": rn, "frame_len": len(fn), "frame_sha256": sha(fn)},
+                           "snappy": {"result": rs, "frame": pack_frame(fs), "chunk_count": list(ref.chunk_count(fs, 0))},
+                           "oracle_snappy_frame": {"result": ro, "frame_sha256": sha(fo),
+                                                   "reference_decode": [rd, sha(data or b""), dfmt]}}
+    G["differential_cpu"] = diff
+    diff = {}
+    for seed in range(10):
+        payload, fmt, k = gpu_differential_case(seed)
+        diff[str(seed)] = {}
+        for name, comp in (("none", HapCompressorNone), ("snappy", HapCompressorSnappy)):
+            r, f = ref.encode([payload], [fmt], [comp], [k])
+            diff[str(seed)][name] = {"result": r, "frame": pack_frame(f), "frame_sha256": sha(f)}
+    G["differential_gpu"] = diff
+
+    # ---- Snappy frames of the picture test_mov_cpu.py hands to FFmpeg (block encoder: tests/twin.py)
+    import twin
+    img = synth.frame(256, 128, 1).numpy()
+    G["mov_frames"] = {}
+    for kind, fmt, chunks in (("bc1", DXT1, 1), ("ycocg", YCOCG, 4)):
+        tex = twin.encode(kind, img)
+        r, f = ref.encode([tex], [fmt], [HapCompressorSnappy], [chunks])
+        assert r == 0
+        G["mov_frames"][kind] = {"frame": pack_frame(f), "payload_sha256": sha(tex)}
 
     out = os.path.join(HERE, "hap_golden.json")
     with open(out, "w") as fh:

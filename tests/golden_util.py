@@ -4,8 +4,12 @@ import functools
 import hashlib
 import json
 import os
+import zlib
 
 import numpy as np
+
+from hap_b200.abi import (HapTextureFormat_A_RGTC1, HapTextureFormat_RGB_DXT1, HapTextureFormat_RGBA_BPTC_UNORM,
+                          HapTextureFormat_RGBA_DXT5, HapTextureFormat_YCoCg_DXT5)
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -34,6 +38,53 @@ def noise_bytes(n, seed=1):
 def kat_c_bytes(n=33177600):
     i = np.arange(n, dtype=np.int64)
     return (((i // 4096) * 3) & 0xFF).astype(np.uint8).tobytes()
+
+
+def pack_frame(frame: bytes) -> str:
+    """How hap_golden.json stores a whole frame: zlib, then base64."""
+    return base64.b64encode(zlib.compress(bytes(frame), 9)).decode()
+
+
+def unpack_frame(s: str) -> bytes:
+    return zlib.decompress(base64.b64decode(s))
+
+
+def dxt_like(rng, blocks, bs):
+    base = rng.integers(0, 256, size=bs * 8, dtype=np.uint8)
+    p = np.tile(base, blocks // 8 + 1)[: blocks * bs].copy()
+    p[:: int(rng.integers(5, 60))] = rng.integers(0, 256)
+    return p.tobytes()
+
+
+DIFFERENTIAL_FORMATS = (HapTextureFormat_RGB_DXT1, HapTextureFormat_YCoCg_DXT5, HapTextureFormat_A_RGTC1,
+                        HapTextureFormat_RGBA_DXT5, HapTextureFormat_RGBA_BPTC_UNORM)
+
+
+def block_bytes(fmt):
+    return 8 if fmt in (HapTextureFormat_RGB_DXT1, HapTextureFormat_A_RGTC1) else 16
+
+
+def cpu_differential_case(seed):
+    """(payload, format, chunk count) of test_oracle_container.py's seeded differential case `seed`: a half-compressible
+    payload of up to 600 blocks."""
+    rng = np.random.default_rng(seed)
+    blocks = int(rng.integers(1, 600))
+    fmt = DIFFERENTIAL_FORMATS[seed % 5]
+    bs = block_bytes(fmt)
+    base = rng.integers(0, 256, size=bs * 4, dtype=np.uint8)
+    payload = np.tile(base, blocks // 4 + 1)[: blocks * bs].copy()
+    payload[:: int(rng.integers(3, 50))] = rng.integers(0, 256)
+    return payload.tobytes(), fmt, int(rng.integers(1, 12))
+
+
+def gpu_differential_case(seed):
+    """(payload, format, chunk count) of test_gpu_parity.py's seeded differential case `seed`: DXT-like bytes, up to
+    40000 blocks."""
+    rng = np.random.default_rng(seed)
+    fmt = DIFFERENTIAL_FORMATS[seed % 5]
+    bs = block_bytes(fmt)
+    payload = dxt_like(rng, int(rng.integers(1, 40000)), bs)
+    return payload, fmt, int(rng.integers(1, 20))
 
 
 def container_checks(lib, decode_kw=None):

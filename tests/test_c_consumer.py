@@ -1,5 +1,6 @@
-"""A compiled C host program that includes the REFERENCE's hap.h (when /root/reference is present; include/hap.h on the
-GPU box, where it is not) and links libhap_b200.so -- the drop-in boundary exercised the way a C application would."""
+"""A compiled C host program that includes the REFERENCE's hap.h (oracle/_ref/c_consumer_ref, built by oracle/Makefile
+where the reference sources are present) or include/hap.h, and links libhap_b200.so -- the drop-in boundary exercised
+the way a C application would."""
 import os
 import subprocess
 
@@ -12,10 +13,11 @@ LIBDIR = os.path.join(ROOT, "hap_b200")
 
 
 def build(which: str) -> str:
-    inc = "/root/reference/source" if which == "ref" else os.path.join(ROOT, "include")
+    if which == "ref":
+        exe = os.path.join(ROOT, "oracle", "_ref", "c_consumer_ref")
+        return exe if os.path.exists(exe) else ""
+    inc = os.path.join(ROOT, "include")
     exe = os.path.join(BUILD, "c_consumer_" + which)
-    if which == "ref" and not os.path.exists(os.path.join(inc, "hap.h")):
-        return exe if os.path.exists(exe) else ""   # built in the container that has the reference; travels with the snapshot
     os.makedirs(BUILD, exist_ok=True)
     subprocess.run(["gcc", "-std=c99", "-O1", "-Wall", "-Werror", "-D_GNU_SOURCE", "-I", inc, SRC, "-o", exe, "-L", LIBDIR,
                     "-l:libhap_b200.so", "-Wl,-rpath," + LIBDIR, "-pthread"], check=True)
@@ -28,7 +30,7 @@ def test_c_consumer_container_paths(which):
     hap_b200.load()
     exe = build(which)
     if not exe:
-        pytest.skip("reference header not present and no prebuilt consumer")
+        pytest.skip("reference build (oracle/_ref) not present")
     p = subprocess.run([exe], capture_output=True, text=True, timeout=120)
     assert p.returncode == 0 and "consumer ok" in p.stdout, p.stdout + p.stderr
 
@@ -38,6 +40,6 @@ def test_c_consumer_container_paths(which):
 def test_c_consumer_gpu_paths(which):
     exe = build(which)
     if not exe:
-        pytest.skip("reference header not present and no prebuilt consumer")
+        pytest.skip("reference build (oracle/_ref) not present")
     p = subprocess.run([exe, "--gpu"], capture_output=True, text=True, timeout=300)
     assert p.returncode == 0 and "GPU paths" in p.stdout, p.stdout + p.stderr

@@ -7,25 +7,18 @@ import torch
 
 import hap_b200
 import oracles
-from golden_util import container_checks, golden, kat_c_bytes, noise_bytes, sha
+from golden_util import container_checks, dxt_like, golden, gpu_differential_case, kat_c_bytes, noise_bytes, sha, unpack_frame
 from hap_b200 import synth
 from hap_b200.abi import (HapCompressorNone, HapCompressorSnappy, HapTextureFormat_A_RGTC1, HapTextureFormat_RGB_DXT1,
-                          HapTextureFormat_RGBA_DXT5, HapTextureFormat_YCoCg_DXT5)
+                          HapTextureFormat_YCoCg_DXT5)
 
 pytestmark = pytest.mark.gpu
-DXT1, DXT5, YCOCG, RGTC1 = HapTextureFormat_RGB_DXT1, HapTextureFormat_RGBA_DXT5, HapTextureFormat_YCoCg_DXT5, HapTextureFormat_A_RGTC1
+DXT1, YCOCG, RGTC1 = HapTextureFormat_RGB_DXT1, HapTextureFormat_YCoCg_DXT5, HapTextureFormat_A_RGTC1
 
 
 @pytest.fixture(scope="module")
 def lib():
     return hap_b200.load()
-
-
-def dxt_like(rng, blocks, bs):
-    base = rng.integers(0, 256, size=bs * 8, dtype=np.uint8)
-    p = np.tile(base, blocks // 8 + 1)[: blocks * bs].copy()
-    p[:: int(rng.integers(5, 60))] = rng.integers(0, 256)
-    return p.tobytes()
 
 
 def test_golden_vectors_of_the_reference(lib):
@@ -77,28 +70,24 @@ def test_encode_kats(lib):
 
 @pytest.mark.parametrize("seed", range(10))
 def test_differential_against_oracle_and_reference(lib, seed):
-    rng = np.random.default_rng(seed)
-    fmt = [DXT1, YCOCG, RGTC1, DXT5, 0x8E8C][seed % 5]
-    bs = 8 if fmt in (DXT1, RGTC1) else 16
-    blocks = int(rng.integers(1, 40000))
-    payload = dxt_like(rng, blocks, bs)
-    k = int(rng.integers(1, 20))
+    payload, fmt, k = gpu_differential_case(seed)
+    G = golden()["differential_gpu"][str(seed)]
     orc, ref = oracles.oracle_abi(), oracles.ref_abi()
-    for comp in (HapCompressorNone, HapCompressorSnappy):
+    for comp, name in ((HapCompressorNone, "none"), (HapCompressorSnappy, "snappy")):
         r, f = lib.encode([payload], [fmt], [comp], [k])
         assert r == 0
         ro, fo = orc.encode([payload], [fmt], [comp], [k])
         if comp == HapCompressorNone:
-            assert f == fo
+            assert f == fo and sha(f) == G[name]["frame_sha256"]      # byte-identical to the reference's frame
         assert lib.chunk_count(f, 0) == orc.chunk_count(fo, 0)
-        for dec in (orc, ref, lib):
+        for dec in (orc, ref, lib):       # ref: the reference build, where it has been built
             if dec is not None:
                 assert dec.decode(f, 0, len(payload))[:3] == (0, payload, fmt)
-        # frames compressed by the oracle (and by Google Snappy through the reference) decode on the GPU
+        # frames compressed by the oracle and (golden) by Google Snappy through the reference decode on the GPU
         assert lib.decode(fo, 0, len(payload))[:3] == (0, payload, fmt)
-        if ref is not None:
-            rr, fr = ref.encode([payload], [fmt], [comp], [k])
-            assert lib.decode(fr, 0, len(payload))[:3] == (0, payload, fmt)
+        fr = unpack_frame(G[name]["frame"])
+        assert G[name]["result"] == 0 and sha(fr) == G[name]["frame_sha256"]
+        assert lib.decode(fr, 0, len(payload))[:3] == (0, payload, fmt)
 
 
 def test_corrupt_streams_never_crash_and_match_oracle_status(lib):

@@ -253,21 +253,26 @@ def test_reader_survives_damaged_movies_under_sanitizers(tmp_path):
 @pytest.mark.parametrize("who", ["oracle", "reference"])
 def test_ffmpeg_decodes_snappy_frames_of_oracle_and_reference(lib, tmp_path, who):
     """Closes the triangle on the CPU: Snappy-compressed, chunked frames written by the oracle port and by the
-    unmodified reference build go through our movie writer and are decoded by FFmpeg's independent Hap decoder to the
-    picture the oracle's block decoder gets from the same texture."""
+    unmodified reference build (stored in tests/golden) go through our movie writer and are decoded by FFmpeg's independent
+    Hap decoder to the picture the oracle's block decoder gets from the same texture."""
     cv2 = pytest.importorskip("cv2")
     import oracles
     import twin
+    from golden_util import golden, sha, unpack_frame
     from hap_b200 import synth
     from hap_b200.abi import HapCompressorSnappy
-    codec = oracles.oracle_abi() if who == "oracle" else oracles.ref_abi()
-    if codec is None:
-        pytest.skip("reference build unavailable")
+    orc = oracles.oracle_abi()
     w, h = 256, 128
     img = synth.frame(w, h, 1).numpy()
     for kind, fmt, cc, chunks in (("bc1", HapTextureFormat_RGB_DXT1, "Hap1", 1), ("ycocg", HapTextureFormat_YCoCg_DXT5, "HapY", 4)):
-        tex = twin.encode(kind, img)
-        r, f = codec.encode([tex], [fmt], [HapCompressorSnappy], [chunks])
+        if who == "oracle":
+            tex = twin.encode(kind, img)
+            r, f = orc.encode([tex], [fmt], [HapCompressorSnappy], [chunks])
+        else:
+            G = golden()["mov_frames"][kind]
+            f = unpack_frame(G["frame"])
+            r, tex, _, _ = orc.decode(f, 0, (w // 4) * (h // 4) * (8 if kind == "bc1" else 16))
+            assert sha(tex) == G["payload_sha256"]
         assert r == 0 and mov.fourcc_for_frame(f) == (0, cc)
         path = str(tmp_path / f"{who}_{cc}.mov")
         with mov.MovWriter(path, cc, w, h, 600) as wr:

@@ -1,10 +1,9 @@
 """Pins the CPU oracle (oracle/hap_oracle.c) against the golden vectors produced by the unmodified
-reference, and differentially against the reference build itself when it is available."""
-import numpy as np
+reference, and checks the reference build itself against them when it is available."""
 import pytest
 
 import oracles
-from golden_util import container_checks, golden, kat_c_bytes, noise_bytes, sha
+from golden_util import container_checks, cpu_differential_case, golden, kat_c_bytes, noise_bytes, sha, unpack_frame
 from hap_b200.abi import (HapCompressorNone, HapCompressorSnappy, HapTextureFormat_A_RGTC1,
                           HapTextureFormat_RGB_DXT1, HapTextureFormat_YCoCg_DXT5)
 
@@ -93,28 +92,19 @@ def test_oracle_encode_argument_results():
 
 @pytest.mark.parametrize("seed", range(6))
 def test_oracle_vs_reference_differential(seed):
-    """Random payloads/chunk counts: None frames byte-identical; Snappy frames cross-decode."""
-    ref = oracles.ref_abi()
-    if ref is None:
-        pytest.skip("reference build unavailable")
+    """Random payloads/chunk counts against the reference's frames of them (golden): None frames byte-identical; Snappy
+    frames cross-decode."""
+    G = golden()["differential_cpu"][str(seed)]
     o = oracles.oracle_abi()
-    rng = np.random.default_rng(seed)
-    blocks = int(rng.integers(1, 600))
-    fmt = [DXT1, YCOCG, RGTC1, 0x83F3, 0x8E8C][seed % 5]
-    bs = 8 if fmt in (DXT1, RGTC1) else 16
-    # half-compressible payload
-    base = rng.integers(0, 256, size=bs * 4, dtype=np.uint8)
-    payload = np.tile(base, blocks // 4 + 1)[: blocks * bs].copy()
-    payload[:: int(rng.integers(3, 50))] = rng.integers(0, 256)
-    payload = payload.tobytes()
-    k = int(rng.integers(1, 12))
-    assert o.max_encoded_length([len(payload)], [fmt], [k]) == ref.max_encoded_length([len(payload)], [fmt], [k])
-    rn, fn = ref.encode([payload], [fmt], [HapCompressorNone], [k])
+    payload, fmt, k = cpu_differential_case(seed)
+    assert o.max_encoded_length([len(payload)], [fmt], [k]) == G["max_len"]
     on, fo = o.encode([payload], [fmt], [HapCompressorNone], [k])
-    assert (rn, fn) == (on, fo)
-    rs, fs = ref.encode([payload], [fmt], [HapCompressorSnappy], [k])
+    assert (on, len(fo), sha(fo)) == (G["none"]["result"], G["none"]["frame_len"], G["none"]["frame_sha256"])
+    fs = unpack_frame(G["snappy"]["frame"])
     os_, fo = o.encode([payload], [fmt], [HapCompressorSnappy], [k])
-    assert rs == os_ == 0
-    assert ref.chunk_count(fs, 0) == o.chunk_count(fo, 0)
-    assert ref.decode(fo, 0, len(payload))[:3] == (0, payload, fmt)
+    assert G["snappy"]["result"] == os_ == 0
+    assert list(o.chunk_count(fo, 0)) == G["snappy"]["chunk_count"]
+    # the reference decoded this very oracle frame to the payload
+    assert sha(fo) == G["oracle_snappy_frame"]["frame_sha256"]
+    assert G["oracle_snappy_frame"]["reference_decode"] == [0, sha(payload), fmt]
     assert o.decode(fs, 0, len(payload))[:3] == (0, payload, fmt)
