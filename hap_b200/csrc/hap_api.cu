@@ -85,6 +85,7 @@ struct DeviceState {
     std::once_flag once;
     bool ready = false;
     int sm_count = 148;
+    int k5_ctas_per_sm = 0;   // resident CTAs of the fragment compressor (K5) per SM
 };
 DeviceState g_dev[kMaxDevices];
 std::atomic<int> g_default_device{-1};
@@ -105,6 +106,12 @@ void device_init(int dev)
     ok = ok && cudaFuncSetAttribute(snappy_index_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(IndexSmem)) == cudaSuccess;
     ok = ok && cudaFuncSetAttribute(snappy_encode_fragments_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)sizeof(EncodeSmem)) == cudaSuccess;
+    ok = ok && cudaFuncSetAttribute(snappy_encode_fragments_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                    (int)cudaSharedmemCarveoutMaxShared) == cudaSuccess;
+    // K5 is built for kEncCtasPerSm resident CTAs (registers, shared memory); a device that fits fewer is not set up
+    ok = ok && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.k5_ctas_per_sm, snappy_encode_fragments_kernel, kEncThreads,
+                                                             sizeof(EncodeSmem)) == cudaSuccess;
+    ok = ok && d.k5_ctas_per_sm >= kEncCtasPerSm;
     if (!ok) { cudaGetLastError(); return; }
     d.ready = true;
 }
@@ -294,11 +301,9 @@ uint32_t launch_encode(const uint8_t *base, const FrameGeom &G, uint32_t frames,
         cudaGetLastError();
         return HapResult_Internal_Error;
     }
-#ifndef HAPB200_ENC_PERSISTENT
-#define HAPB200_ENC_PERSISTENT 1
-#endif
-    // one resident CTA per SM strides over the fragments (the kernel's 131 KB of shared memory allow no second one)
-    const unsigned k5_grid = HAPB200_ENC_PERSISTENT ? (unsigned)(nfrag < (uint64_t)sm_count() ? nfrag : (uint64_t)sm_count()) : (unsigned)nfrag;
+    // every resident CTA slot of the device strides over the fragments (two CTAs of 512 threads per SM)
+    const uint64_t k5_slots = (uint64_t)g_dev[t_device].k5_ctas_per_sm * (uint64_t)sm_count();
+    const unsigned k5_grid = (unsigned)(nfrag < k5_slots ? nfrag : k5_slots);
     HAP_KLAUNCH(kStSnappyEncode, snappy_encode_fragments_kernel, dim3(k5_grid), dim3(kEncThreads), sizeof(EncodeSmem), st, base, G,
                 (uint32_t)nfrag, scratch.as<uint8_t>(), fsize.as<uint32_t>(), write_index ? fent.as<uint8_t>() : (uint8_t *)nullptr);
     HAP_KLAUNCH(kStPlan, hap_plan_frames_kernel, dim3(frames), dim3(kPlanThreads), 0, st, G, base, fsize.as<uint32_t>(),

@@ -4,7 +4,7 @@
 // (/root/reference/source/hap.c:448-476, call site :453).  The reference's loop is serial over chunks
 // and Snappy is serial inside a chunk; here a chunk is cut into independent 32 KiB FRAGMENTS (a raw
 // Snappy stream is varint(length) followed by elements, so fragment element streams concatenate
-// into one legal chunk stream as long as copies never reach outside their fragment), one resident CTA
+// into one legal chunk stream as long as copies never reach outside their fragment), two resident CTAs
 // per SM striding over the fragments, and inside a fragment every 8-byte unit is handled on its own:
 //   1. first-occurrence hash of every aligned word (shared-memory table, atomicMin => deterministic);
 //   2. each word picks a source: the word one DXT block back when its whole block repeats the
@@ -23,8 +23,9 @@
 
 namespace hapb200 {
 
-constexpr int kEncThreads = 1024;
+constexpr int kEncThreads = 512;
 constexpr int kEncWarps = kEncThreads / 32;
+constexpr int kEncCtasPerSm = 2;            // resident CTAs per SM the kernel is built for (registers and shared memory)
 constexpr int kFragBytes = 32768;
 constexpr int kFragCap = kFragBytes + 32;   // element stream of a fragment never exceeds n + 3
 constexpr int kEncHashBits = 13;
@@ -33,26 +34,34 @@ constexpr int kFragEntryPieces = (kFragCap + (1 << kIndexSubLog2) - 1) >> kIndex
 constexpr int kFragEntryStride = 272;             // bytes reserved per fragment in the entries scratch (multiple of 16)
 static_assert(kFragEntryPieces <= kFragEntryStride, "entries of one fragment fit their scratch slot");
 
-// Shared memory of one fragment.  The unit of every decision is 8 BYTES (a DXT1 / RGTC1 block, half a DXT5 block): thread t
-// owns the 4 consecutive units [4t, 4t+4) and keeps them (and every per-unit quantity) in registers; shared memory only
+// Shared memory of one fragment.  The unit of every decision is 8 BYTES (a DXT1 / RGTC1 block, half a DXT5 block).  Units are
+// grouped in STRIPS of 4 consecutive units; thread t owns the two strips t and t + kEncThreads, i.e. units [4t, 4t+4) and
+// [4t + kHalfUnits, 4t + kHalfUnits + 4), and keeps them (and every per-unit quantity) in registers.  Shared memory only
 // carries what OTHER threads read: the data (random match verification), the hash table, the strip-boundary values of the
-// per-unit arrays, and -- for the last step, which re-distributes the units over the threads -- positions, run starts and
-// distances.  (Round 1 decided per 4-byte word: twice the elements in every step, and 4-byte matches that were demoted
-// again because a copy element costs 3 bytes.  Matches that start at an odd word are lost; DXT payloads hardly have any.)
+// per-unit arrays, and -- for the last step, which re-distributes the units over the threads -- positions and run starts.
+// (Round 1 decided per 4-byte word: twice the elements in every step, and 4-byte matches that were demoted again because a
+// copy element costs 3 bytes.  Matches that start at an odd word are lost; DXT payloads hardly have any.)
+// Two CTAs share an SM, so that one CTA's barrier drains are filled by the other's work.  To fit two, the output step's
+// arrays (positions, run starts and the element stream) overlay the hash table, which is dead by then.  (Overlaying the
+// element stream on the input units instead, with the output step reading its literal bytes from global memory, was
+// measured: K5 5.35 ms per 444 4K Hap Q frames against 5.64 with one 1024-thread CTA -- eight dependent L2 reads per
+// thread in the output loop ate most of what the second CTA brings.)
 #ifndef HAPB200_K5_ROUNDS
 #define HAPB200_K5_ROUNDS 1
 #endif
 constexpr int kFragUnits = kFragBytes / 8;        // 4096
-constexpr int kUnitStrip = kFragUnits / kEncThreads;   // 4 units per thread
-static_assert(kUnitStrip == 4, "the strip code below moves 4 uint16 values per thread as one 8-byte access");
+constexpr int kUnitStrip = 4;                     // units per strip
+constexpr int kEncStrips = kFragUnits / (kUnitStrip * kEncThreads);   // strips per thread
+constexpr int kHalfUnits = kUnitStrip * kEncThreads;                  // units of all threads' first strips (2048)
+static_assert(kEncStrips == 2, "a thread owns two strips: the block scans carry the two halves of the fragment as one packed word");
 struct EncodeSmem {
     uint2 data[kFragUnits + 2];                     // input units
     union {
-        uint32_t table[1 << kEncHashBits];          // first occurrence of every hashed unit
+        uint32_t table[1 << kEncHashBits];          // first occurrence of every hashed unit (steps 1 .. 2)
         struct {
-            uint16_t a[kFragUnits];                 // final distance per unit (read by the re-dealt output step)
-            uint16_t b[kFragUnits];                 // run start per unit
-            uint16_t c[kFragUnits];                 // stream position per unit
+            uint16_t b[kFragUnits];                 // run start per unit (step 5)
+            uint16_t c[kFragUnits];                 // stream position per unit (step 5)
+            alignas(16) uint32_t out[(kFragCap + 3) / 4 + 6];   // the element stream (step 5, copied out in 16-byte words)
         } h;
     } u;
     uint16_t da[kFragUnits];                        // candidate distances (ping) | one of the two holds the final distances,
@@ -60,8 +69,9 @@ struct EncodeSmem {
     uint32_t warp_tot[kEncWarps];
     uint32_t entry[kFragEntryStride];               // fragment index: offset of the first element start in every 128 bytes of the stream
     uint32_t total;
-    alignas(16) uint32_t out[(kFragCap + 3) / 4 + 6];   // the element stream (copied out in 16-byte words)
 };
+// Two resident CTAs: 233,472 B of shared memory per SM, of which every CTA reserves 1 KiB for the system.
+static_assert(sizeof(EncodeSmem) <= 233472 / kEncCtasPerSm - 1024, "two K5 CTAs fit one SM's shared memory");
 
 __device__ __forceinline__ uint32_t enc_hash(uint2 u) { return ((u.x * 0x9E3779B1u) ^ (u.y * 0x85EBCA6Bu)) >> (32 - kEncHashBits); }
 __device__ __forceinline__ bool same_unit(uint2 a, uint2 b) { return a.x == b.x && a.y == b.y; }
@@ -73,187 +83,244 @@ __device__ __forceinline__ void store_strip16(uint16_t *arr, uint32_t base, cons
     *reinterpret_cast<uint2 *>(arr + base) = make_uint2(v[0] | (v[1] << 16), v[2] | (v[3] << 16));
 }
 
-// Inclusive max / sum over the block of one value per thread; returns the exclusive prefix for this thread and
-// the block total.  Two barriers.  The 32 warp totals are scanned by every warp with shuffles (lane w holds the
-// total of warp w) instead of a 32-step loop over shared memory.
+// Per-half max of two 16-bit values packed in one word (the block scans below carry both halves of a fragment at once).
+__device__ __forceinline__ uint32_t enc_max_u16x2(uint32_t a, uint32_t b)
+{
+#ifdef HAPB200_EMU
+    const uint32_t lo = (a & 0xFFFFu) > (b & 0xFFFFu) ? (a & 0xFFFFu) : (b & 0xFFFFu), hi = (a >> 16) > (b >> 16) ? (a >> 16) : (b >> 16);
+    return lo | (hi << 16);
+#else
+    return __vmaxu2(a, b);
+#endif
+}
+
+// Inclusive max / sum over the block of one PACKED value per thread (two 16-bit halves, scanned independently: a sum
+// never carries out of the low half because every half-fragment total stays below 2^16); returns the exclusive prefix
+// for this thread and the block total, both packed.  Two barriers.  The warp totals are scanned by every warp with
+// shuffles (lane w holds the total of warp w) instead of a loop over shared memory.
 __device__ __forceinline__ uint32_t enc_block_excl(uint32_t v, bool is_max, uint32_t *total, uint32_t *warp_tot)
 {
-    static_assert(kEncWarps == 32, "one warp total per lane");
+    static_assert(kEncWarps <= 32 && (kEncWarps & (kEncWarps - 1)) == 0, "one warp total per lane");
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     uint32_t incl = v;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
         uint32_t o = __shfl_up_sync(HAP_FULL_MASK, incl, d);
-        if (lane >= d) incl = is_max ? (incl > o ? incl : o) : incl + o;
+        if (lane >= d) incl = is_max ? enc_max_u16x2(incl, o) : incl + o;
     }
     uint32_t prev = __shfl_up_sync(HAP_FULL_MASK, incl, 1);
     if (lane == 0) prev = 0;
     if (lane == 31) warp_tot[warp] = incl;
     __syncthreads();
-    uint32_t wi = warp_tot[lane];
+    uint32_t wi = lane < kEncWarps ? warp_tot[lane] : 0u;   // (0 is the identity of both operations)
 #pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
+    for (int d = 1; d < kEncWarps; d <<= 1) {
         uint32_t o = __shfl_up_sync(HAP_FULL_MASK, wi, d);
-        if (lane >= d) wi = is_max ? (wi > o ? wi : o) : wi + o;
+        if (lane >= d) wi = is_max ? enc_max_u16x2(wi, o) : wi + o;
     }
-    const uint32_t tot = __shfl_sync(HAP_FULL_MASK, wi, 31);
+    const uint32_t tot = __shfl_sync(HAP_FULL_MASK, wi, kEncWarps - 1);
     uint32_t base = __shfl_sync(HAP_FULL_MASK, wi, warp > 0 ? warp - 1 : 0);
     if (warp == 0) base = 0;
     __syncthreads();
     *total = tot;
-    return is_max ? (base > prev ? base : prev) : base + prev;
+    return is_max ? enc_max_u16x2(base, prev) : base + prev;
 }
 
-// One fragment: U units (8 bytes each; U <= kFragUnits) already in S.data AND in the caller's registers d[4] (units
-// 4t..4t+3) -> element stream written to S.out as bytes; returns its size (all threads).
+// One fragment: U units (8 bytes each; U <= kFragUnits) already in S.data AND in the caller's registers d[8] (units
+// 4t..4t+3, then kHalfUnits+4t..kHalfUnits+4t+3) -> element stream written to S.u.h.out as bytes; returns its size (all
+// threads).
 // period_units = DXT block size in units (1 or 2).
 // FULL = the fragment has all kFragUnits units (31 of 32 fragments of a 1 MiB chunk): every per-unit bounds test
 // folds away at compile time.
+// Every decision below is a rule over unit indices (atomicMin, one Jacobi round of propagation, max and sum scans in unit
+// order), so the stream does not depend on which thread owns which unit.
 template <bool FULL>
-__device__ __forceinline__ uint32_t compress_fragment(EncodeSmem &S, const uint2 d[4], uint32_t Udyn, uint32_t period_units)
+__device__ __forceinline__ uint32_t compress_fragment(EncodeSmem &S, const uint2 d[8], uint32_t Udyn, uint32_t period_units)
 {
+    constexpr int kUnitsPerThread = kEncStrips * kUnitStrip;
     const uint32_t t = threadIdx.x;
     const uint32_t U = FULL ? (uint32_t)kFragUnits : Udyn;
-    const uint32_t i0 = t * kUnitStrip;              // first unit of my strip
-    const uint32_t nv = FULL ? (uint32_t)kUnitStrip : (i0 >= U ? 0u : (U - i0 < (uint32_t)kUnitStrip ? U - i0 : (uint32_t)kUnitStrip));  // my valid units
+    uint32_t i0[kEncStrips], nv[kEncStrips];       // first unit of each of my strips, and its valid units
+#pragma unroll
+    for (int h = 0; h < kEncStrips; h++) {
+        i0[h] = h * kHalfUnits + t * kUnitStrip;
+        nv[h] = FULL ? (uint32_t)kUnitStrip : (i0[h] >= U ? 0u : (U - i0[h] < (uint32_t)kUnitStrip ? U - i0[h] : (uint32_t)kUnitStrip));
+    }
 
     // 1. first occurrence of every unit (the table was initialised by the caller, before the barrier)
-    uint32_t hsh[4];
+    uint32_t hsh[kUnitsPerThread];
 #pragma unroll
-    for (int k = 0; k < kUnitStrip; k++) {
-        hsh[k] = enc_hash(d[k]);
-        if ((uint32_t)k < nv) atomicMin(&S.u.table[hsh[k]], i0 + k);
-    }
+    for (int h = 0; h < kEncStrips; h++)
+#pragma unroll
+        for (int k = 0; k < kUnitStrip; k++) {
+            hsh[h * kUnitStrip + k] = enc_hash(d[h * kUnitStrip + k]);
+            if ((uint32_t)k < nv[h]) atomicMin(&S.u.table[hsh[h * kUnitStrip + k]], i0[h] + k);
+        }
     __syncthreads();
 
     // 2. candidate distance per unit: first earlier occurrence, or one block back when the whole block repeats
-    uint32_t dd[4];
+    uint32_t dd[kUnitsPerThread];
 #pragma unroll
-    for (int k = 0; k < kUnitStrip; k++) {
-        dd[k] = 0;
-        if ((uint32_t)k < nv) {
-            const uint32_t c = S.u.table[hsh[k]];
-            if (c < i0 + k && same_unit(S.data[c], d[k])) dd[k] = i0 + k - c;
+    for (int h = 0; h < kEncStrips; h++) {
+        const uint2 *dh = d + h * kUnitStrip;
+        uint32_t *ddh = dd + h * kUnitStrip;
+        const uint32_t s0 = i0[h];
+#pragma unroll
+        for (int k = 0; k < kUnitStrip; k++) {
+            ddh[k] = 0;
+            if ((uint32_t)k < nv[h]) {
+                const uint32_t c = S.u.table[hsh[h * kUnitStrip + k]];
+                if (c < s0 + k && same_unit(S.data[c], dh[k])) ddh[k] = s0 + k - c;
+            }
         }
-    }
-    if (period_units == 2) {
-        // DXT5-sized blocks: units (2b, 2b+1); the block repeats when both units equal the block before
-        const uint2 p0 = i0 >= 2 ? S.data[i0 - 2] : make_uint2(0, 0), p1 = i0 >= 2 ? S.data[i0 - 1] : make_uint2(0, 0);
-        if (i0 >= 2 && nv >= 2 && same_unit(p0, d[0]) && same_unit(p1, d[1])) { dd[0] = 2; dd[1] = 2; }
-        if (nv >= 4 && same_unit(d[0], d[2]) && same_unit(d[1], d[3])) { dd[2] = 2; dd[3] = 2; }
-    } else {
-        const uint2 p = i0 >= 1 ? S.data[i0 - 1] : make_uint2(0, 0);
-        if (i0 >= 1 && nv >= 1 && same_unit(p, d[0])) dd[0] = 1;
+        if (period_units == 2) {
+            // DXT5-sized blocks: units (2b, 2b+1); the block repeats when both units equal the block before
+            const uint2 p0 = s0 >= 2 ? S.data[s0 - 2] : make_uint2(0, 0), p1 = s0 >= 2 ? S.data[s0 - 1] : make_uint2(0, 0);
+            if (s0 >= 2 && nv[h] >= 2 && same_unit(p0, dh[0]) && same_unit(p1, dh[1])) { ddh[0] = 2; ddh[1] = 2; }
+            if (nv[h] >= 4 && same_unit(dh[0], dh[2]) && same_unit(dh[1], dh[3])) { ddh[2] = 2; ddh[3] = 2; }
+        } else {
+            const uint2 p = s0 >= 1 ? S.data[s0 - 1] : make_uint2(0, 0);
+            if (s0 >= 1 && nv[h] >= 1 && same_unit(p, dh[0])) ddh[0] = 1;
 #pragma unroll
-        for (int k = 1; k < kUnitStrip; k++)
-            if ((uint32_t)k < nv && same_unit(d[k - 1], d[k])) dd[k] = 1;
+            for (int k = 1; k < kUnitStrip; k++)
+                if ((uint32_t)k < nv[h] && same_unit(dh[k - 1], dh[k])) ddh[k] = 1;
+        }
+        store_strip16(S.da, s0, ddh);
     }
-    store_strip16(S.da, i0, dd);
     __syncthreads();
 
-    // 2b. propagation (two rounds): a unit that is not yet part of a run adopts its left (else right) neighbour's
-    //     distance when its own data also matches there.  First occurrences of neighbouring units often point at
-    //     different earlier blocks; this re-aligns them and recovers most of what a greedy match extension finds.
+    // 2b. propagation: a unit that is not yet part of a run adopts its left (else right) neighbour's distance when its own
+    //     data also matches there.  First occurrences of neighbouring units often point at different earlier blocks; this
+    //     re-aligns them and recovers most of what a greedy match extension finds.
     uint16_t *cur = S.da, *nxt = S.db;
     {
 #pragma unroll 1
         for (int round = 0; round < HAPB200_K5_ROUNDS; round++) {
-            const uint32_t lb = i0 > 0 ? cur[i0 - 1] : 0u;
-            const uint32_t rb = i0 + kUnitStrip < U ? cur[i0 + kUnitStrip] : 0u;
-            uint32_t nd[4];
+            uint32_t nd[kUnitsPerThread];
 #pragma unroll
-            for (int k = 0; k < kUnitStrip; k++) {
-                const uint32_t l = k > 0 ? dd[k - 1] : lb, r = k < kUnitStrip - 1 ? dd[k + 1] : rb;
-                const uint32_t cd = dd[k], i = i0 + k;
-                nd[k] = cd;
-                if ((uint32_t)k < nv && !(cd != 0 && (cd == l || cd == r))) {
-                    // one look-up decides: the left neighbour's distance if there is one, else the right one's
-                    const uint32_t cand = l != 0 ? l : r;
-                    if (cand != 0 && i >= cand && same_unit(S.data[i - cand], d[k])) nd[k] = cand;
-                    else if (l != 0 && r != 0 && r != l && i >= r && same_unit(S.data[i - r], d[k])) nd[k] = r;
+            for (int h = 0; h < kEncStrips; h++) {
+                const uint32_t s0 = i0[h];
+                const uint32_t lb = s0 > 0 ? cur[s0 - 1] : 0u;
+                const uint32_t rb = s0 + kUnitStrip < U ? cur[s0 + kUnitStrip] : 0u;
+#pragma unroll
+                for (int k = 0; k < kUnitStrip; k++) {
+                    const int u = h * kUnitStrip + k;
+                    const uint32_t l = k > 0 ? dd[u - 1] : lb, r = k < kUnitStrip - 1 ? dd[u + 1] : rb;
+                    const uint32_t cd = dd[u], i = s0 + k;
+                    nd[u] = cd;
+                    if ((uint32_t)k < nv[h] && !(cd != 0 && (cd == l || cd == r))) {
+                        // one look-up decides: the left neighbour's distance if there is one, else the right one's
+                        const uint32_t cand = l != 0 ? l : r;
+                        if (cand != 0 && i >= cand && same_unit(S.data[i - cand], d[u])) nd[u] = cand;
+                        else if (l != 0 && r != 0 && r != l && i >= r && same_unit(S.data[i - r], d[u])) nd[u] = r;
+                    }
                 }
             }
 #pragma unroll
-            for (int k = 0; k < kUnitStrip; k++) dd[k] = nd[k];
-            store_strip16(nxt, i0, dd);
+            for (int u = 0; u < kUnitsPerThread; u++) dd[u] = nd[u];
+#pragma unroll
+            for (int h = 0; h < kEncStrips; h++) store_strip16(nxt, i0[h], dd + h * kUnitStrip);
             __syncthreads();
             uint16_t *tmp = cur; cur = nxt; nxt = tmp;
         }
     }
-    // `cur` holds the final distances (read across strip boundaries below); the other buffer is free: it takes the run ends.
+    // `cur` holds the final distances (read across strip boundaries below, and by the output step); the other buffer is
+    // free: it takes the run ends.
     // (Measured on the emulator cases: with 8-byte units ONE round recovers what two did -- frame sizes equal on picture
     // content, +0.1 .. 0.5 % on the stitched random cases; none costs 5 .. 16 %.)
     const uint16_t *fin = cur;
     uint16_t *ends = nxt;
     // (a single matching unit is kept: an 8-byte copy costs 3 bytes)
-    store_strip16(S.u.h.a, i0, dd);   // the hash table is dead: its space holds the final distances
 
     // 3. run start of every unit (max-scan of "i+1 where a run starts") and run ends (stored at the run start)
-    uint32_t rs[4];
+    uint32_t rs[kUnitsPerThread];
     {
-        const uint32_t lb = i0 > 0 ? fin[i0 - 1] : 0u;
-        uint32_t last = 0;  // (index + 1) of the last run start inside my strip so far
-        uint32_t loc[4];
+        uint32_t last[kEncStrips];  // (index + 1) of the last run start inside each strip so far
+        uint32_t loc[kUnitsPerThread];
 #pragma unroll
-        for (int k = 0; k < kUnitStrip; k++) {
-            const uint32_t prev = k > 0 ? dd[k - 1] : lb;
-            if ((uint32_t)k < nv && (i0 + k == 0 || dd[k] != prev)) last = i0 + k + 1;
-            loc[k] = last;
+        for (int h = 0; h < kEncStrips; h++) {
+            const uint32_t s0 = i0[h];
+            const uint32_t lb = s0 > 0 ? fin[s0 - 1] : 0u;
+            last[h] = 0;
+#pragma unroll
+            for (int k = 0; k < kUnitStrip; k++) {
+                const int u = h * kUnitStrip + k;
+                const uint32_t prev = k > 0 ? dd[u - 1] : lb;
+                if ((uint32_t)k < nv[h] && (s0 + k == 0 || dd[u] != prev)) last[h] = s0 + k + 1;
+                loc[u] = last[h];
+            }
         }
-        uint32_t unused;
-        const uint32_t carry = enc_block_excl(last, true, &unused, S.warp_tot);
+        uint32_t tot;
+        const uint32_t ex = enc_block_excl(last[0] | (last[1] << 16), true, &tot, S.warp_tot);
+        // strips of the second half follow every strip of the first half in unit order
+        const uint32_t carry[kEncStrips] = {ex & 0xFFFFu, (tot & 0xFFFFu) > (ex >> 16) ? (tot & 0xFFFFu) : (ex >> 16)};
 #pragma unroll
-        for (int k = 0; k < kUnitStrip; k++) rs[k] = (loc[k] ? loc[k] : carry) - 1;
-        const uint32_t rb = i0 + kUnitStrip < U ? fin[i0 + kUnitStrip] : 0xFFFFFFFFu;
+        for (int u = 0; u < kUnitsPerThread; u++) rs[u] = (loc[u] ? loc[u] : carry[u / kUnitStrip]) - 1;
 #pragma unroll
-        for (int k = 0; k < kUnitStrip; k++) {
-            const uint32_t nx = k < kUnitStrip - 1 ? dd[k + 1] : rb;
-            if ((uint32_t)k < nv && (i0 + k + 1 == U || nx != dd[k])) ends[rs[k]] = (uint16_t)(i0 + k);
+        for (int h = 0; h < kEncStrips; h++) {
+            const uint32_t s0 = i0[h];
+            const uint32_t rb = s0 + kUnitStrip < U ? fin[s0 + kUnitStrip] : 0xFFFFFFFFu;
+#pragma unroll
+            for (int k = 0; k < kUnitStrip; k++) {
+                const int u = h * kUnitStrip + k;
+                const uint32_t nx = k < kUnitStrip - 1 ? dd[u + 1] : rb;
+                if ((uint32_t)k < nv[h] && (s0 + k + 1 == U || nx != dd[u])) ends[rs[u]] = (uint16_t)(s0 + k);
+            }
         }
     }
     __syncthreads();
 
     // 4. bytes each unit contributes and their exclusive prefix sum
-    uint32_t pos[4];
+    uint32_t pos[kUnitsPerThread];
     {
-        uint32_t run = 0;
+        uint32_t run[kEncStrips];
 #pragma unroll
-        for (int k = 0; k < kUnitStrip; k++) {
-            uint32_t c = 0;
-            if ((uint32_t)k < nv) {
-                const uint32_t i = i0 + k;
-                if (dd[k] == 0) {
-                    c = 8;
-                    if (i == rs[k]) c += literal_header_bytes(8u * (ends[i] - i + 1));
-                } else if (((i - rs[k]) & 7) == 0) {
-                    c = 3;      // one copy element per 64 bytes of the run
+        for (int h = 0; h < kEncStrips; h++) {
+            run[h] = 0;
+#pragma unroll
+            for (int k = 0; k < kUnitStrip; k++) {
+                const int u = h * kUnitStrip + k;
+                uint32_t c = 0;
+                if ((uint32_t)k < nv[h]) {
+                    const uint32_t i = i0[h] + k;
+                    if (dd[u] == 0) {
+                        c = 8;
+                        if (i == rs[u]) c += literal_header_bytes(8u * (ends[i] - i + 1));
+                    } else if (((i - rs[u]) & 7) == 0) {
+                        c = 3;      // one copy element per 64 bytes of the run
+                    }
                 }
+                pos[u] = run[h];
+                run[h] += c;
             }
-            pos[k] = run;
-            run += c;
         }
         uint32_t tot;
-        const uint32_t base = enc_block_excl(run, false, &tot, S.warp_tot);
+        const uint32_t ex = enc_block_excl(run[0] | (run[1] << 16), false, &tot, S.warp_tot);
+        const uint32_t base[kEncStrips] = {ex & 0xFFFFu, (tot & 0xFFFFu) + (ex >> 16)};
 #pragma unroll
-        for (int k = 0; k < kUnitStrip; k++) pos[k] += base;
-        if (t == 0) S.total = tot;
+        for (int u = 0; u < kUnitsPerThread; u++) pos[u] += base[u / kUnitStrip];
+        if (t == 0) S.total = (tot & 0xFFFFu) + (tot >> 16);
     }
 
-    // 5. every unit writes its own bytes.  Ownership changes for this step: thread t takes units t, t + 1024, ... so that
-    //    the lanes of a warp write neighbouring bytes of the stream (with the strip layout they sit 32 bytes apart: bank
-    //    conflicts on every store).  Positions, run starts and distances travel through shared memory as 16-bit strips.
+    // 5. every unit writes its own bytes.  Ownership changes for this step: thread t takes units t, t + kEncThreads, ... so
+    //    that the lanes of a warp write neighbouring bytes of the stream (with the strip layout they sit 32 bytes apart: bank
+    //    conflicts on every store).  Positions and run starts travel through shared memory as 16-bit strips, the distances
+    //    are the final ones of step 2b.
     //    Inside a literal run the stream is the input shifted by (p & 3) bytes, so a unit writes TWO aligned 32-bit words
     //    made of its own bytes and the next unit's first bytes; only the two ends of a run, headers and copy elements are
     //    written bytewise.
-    store_strip16(S.u.h.c, i0, pos);
-    store_strip16(S.u.h.b, i0, rs);
+#pragma unroll
+    for (int h = 0; h < kEncStrips; h++) {
+        store_strip16(S.u.h.c, i0[h], pos + h * kUnitStrip);
+        store_strip16(S.u.h.b, i0[h], rs + h * kUnitStrip);
+    }
     __syncthreads();
-    uint8_t *out = reinterpret_cast<uint8_t *>(S.out);
+    uint8_t *out = reinterpret_cast<uint8_t *>(S.u.h.out);
 #pragma unroll 1
-    for (int j = 0; j < kUnitStrip; j++) {
+    for (int j = 0; j < kUnitsPerThread; j++) {
         const uint32_t i = t + (uint32_t)j * kEncThreads;
         if (!FULL && i >= U) continue;
-        const uint32_t dist = S.u.h.a[i], rs_i = S.u.h.b[i];
+        const uint32_t dist = fin[i], rs_i = S.u.h.b[i];
         uint32_t p = S.u.h.c[i];
         if (dist == 0) {
             const uint2 w = S.data[i];
@@ -366,7 +433,7 @@ __device__ __forceinline__ FragRef locate_fragment(const uint8_t *dxt, const Fra
     return r;
 }
 
-// A thread's 4 units of a fragment, from global memory: two 16-byte loads when possible
+// A strip of 4 units of a fragment, from global memory: two 16-byte loads when possible
 __device__ __forceinline__ void load_strip(const FragRef &fr, uint32_t i0, uint2 d[4])
 {
     if ((((uintptr_t)fr.in) & 15) == 0 && i0 + kUnitStrip <= fr.units) {
@@ -387,63 +454,51 @@ __device__ __forceinline__ void load_strip(const FragRef &fr, uint32_t i0, uint2
     }
 }
 
-// A fixed grid (one CTA per SM: the kernel needs 123 KB of shared memory) strides over the nfrag = frames *
-// frags_per_frame fragments of the batch.  A thread's units of the NEXT fragment are loaded before the current one is
-// compressed, so the HBM latency of the input and the turn-over between CTAs -- both fully exposed with a single CTA
-// per SM -- are covered by a fragment's worth of work.
+// A fixed grid (kEncCtasPerSm resident CTAs per SM) strides over the nfrag = frames * frags_per_frame fragments of the
+// batch.  The HBM latency of a fragment's input and the turn-over between fragments are covered by the other CTA on the
+// same SM, which is at a different phase of its own fragment.
 // dxt: base pointer of the texture bytes; scratch: [nfrag][kFragCap]; frag_size: [nfrag] (kFragStoredRaw when the
 // fragment was not compressed); frag_entries: [nfrag][kFragEntryStride] or nullptr (fragment index, hap_index.h).
-__global__ void __launch_bounds__(kEncThreads) snappy_encode_fragments_kernel(
+__global__ void __launch_bounds__(kEncThreads, kEncCtasPerSm) snappy_encode_fragments_kernel(
     const uint8_t *__restrict__ dxt, FrameGeom G, uint32_t nfrag, uint8_t *__restrict__ scratch, uint32_t *__restrict__ frag_size,
     uint8_t *__restrict__ frag_entries)
 {
     HAP_DYN_SMEM(smem_raw);
     EncodeSmem &S = *reinterpret_cast<EncodeSmem *>(smem_raw);
     const int t = threadIdx.x;
-    const uint32_t i0 = (uint32_t)t * kUnitStrip;
-    uint32_t gfrag = blockIdx.x;
-    if (gfrag >= nfrag) return;
-    FragRef cur = locate_fragment(dxt, G, gfrag);
-    uint2 d[4];
-    load_strip(cur, i0, d);
-    for (;;) {
-        const uint32_t next = gfrag + gridDim.x;
-        FragRef nxt;
-        uint2 nd[4];
-        const bool more = next < nfrag;
-        if (more) {
-            nxt = locate_fragment(dxt, G, next);
-            load_strip(nxt, i0, nd);     // in flight while this fragment is compressed
-        }
+    for (uint32_t gfrag = blockIdx.x; gfrag < nfrag; gfrag += gridDim.x) {
+        const FragRef cur = locate_fragment(dxt, G, gfrag);
         if (cur.units == 0) {
             if (t == 0) frag_size[gfrag] = kFragStoredRaw;
-        } else {
-            const uint32_t U = cur.units;
-            *reinterpret_cast<uint4 *>(&S.data[i0]) = make_uint4(d[0].x, d[0].y, d[1].x, d[1].y);
-            *reinterpret_cast<uint4 *>(&S.data[i0 + 2]) = make_uint4(d[2].x, d[2].y, d[3].x, d[3].y);
-            {
-                uint4 *tb = reinterpret_cast<uint4 *>(S.u.table);
-                const uint4 ones = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
-                for (int q = t; q < (1 << kEncHashBits) / 4; q += kEncThreads) tb[q] = ones;
-                if (t < kFragEntryStride) S.entry[t] = kIndexNoEntry;
-            }
-            __syncthreads();
-            const uint32_t period_units = (cur.second ? G.s[1].period_words : G.s[0].period_words) >> 1;   // 8-byte blocks: 1, 16-byte blocks: 2
-            const uint32_t total = U == (uint32_t)kFragUnits ? compress_fragment<true>(S, d, U, period_units)
-                                                             : compress_fragment<false>(S, d, U, period_units);
-            uint8_t *o = scratch + (uint64_t)gfrag * kFragCap;
-            const uint4 *o4s = reinterpret_cast<const uint4 *>(S.out);
-            uint4 *o4 = reinterpret_cast<uint4 *>(o);       // (scratch slots are kFragCap = 32800 bytes apart: 16-byte aligned)
-            for (uint32_t i = t; i < (total + 15) / 16; i += kEncThreads) o4[i] = o4s[i];
-            if (frag_entries != nullptr && t < kFragEntryStride) frag_entries[(uint64_t)gfrag * kFragEntryStride + t] = (uint8_t)S.entry[t];
-            if (t == 0) frag_size[gfrag] = total;
-            __syncthreads();   // S.out, S.data and the tables are rewritten by the next fragment
+            continue;
         }
-        if (!more) break;
-        gfrag = next;
-        cur = nxt;
+        const uint32_t U = cur.units;
+        uint2 d[kEncStrips * kUnitStrip];
 #pragma unroll
-        for (int k = 0; k < kUnitStrip; k++) d[k] = nd[k];
+        for (int h = 0; h < kEncStrips; h++) {
+            const uint32_t i0 = h * kHalfUnits + (uint32_t)t * kUnitStrip;
+            uint2 *dh = d + h * kUnitStrip;
+            load_strip(cur, i0, dh);
+            *reinterpret_cast<uint4 *>(&S.data[i0]) = make_uint4(dh[0].x, dh[0].y, dh[1].x, dh[1].y);
+            *reinterpret_cast<uint4 *>(&S.data[i0 + 2]) = make_uint4(dh[2].x, dh[2].y, dh[3].x, dh[3].y);
+        }
+        {
+            uint4 *tb = reinterpret_cast<uint4 *>(S.u.table);
+            const uint4 ones = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu);
+            for (int q = t; q < (1 << kEncHashBits) / 4; q += kEncThreads) tb[q] = ones;
+            if (t < kFragEntryStride) S.entry[t] = kIndexNoEntry;
+        }
+        __syncthreads();
+        const uint32_t period_units = (cur.second ? G.s[1].period_words : G.s[0].period_words) >> 1;   // 8-byte blocks: 1, 16-byte blocks: 2
+        const uint32_t total = U == (uint32_t)kFragUnits ? compress_fragment<true>(S, d, U, period_units)
+                                                         : compress_fragment<false>(S, d, U, period_units);
+        uint8_t *o = scratch + (uint64_t)gfrag * kFragCap;
+        const uint4 *o4s = reinterpret_cast<const uint4 *>(S.u.h.out);
+        uint4 *o4 = reinterpret_cast<uint4 *>(o);       // (scratch slots are kFragCap = 32800 bytes apart: 16-byte aligned)
+        for (uint32_t i = t; i < (total + 15) / 16; i += kEncThreads) o4[i] = o4s[i];
+        if (frag_entries != nullptr && t < kFragEntryStride) frag_entries[(uint64_t)gfrag * kFragEntryStride + t] = (uint8_t)S.entry[t];
+        if (t == 0) frag_size[gfrag] = total;
+        __syncthreads();   // S.data and the tables (with the element stream) are rewritten by the next fragment
     }
 }
 
